@@ -14,6 +14,9 @@ bandwidth; `roofline.bwt_stage` is the whole forward BWT.  Further objects on th
 `parity` (oracle vs the first blocks of the benchmarked stream), `decode` (resident + end to end +
 roofline), `config3` (100 MB enwik-shaped text, encode + decode), `bwtc` (BASELINE configs[3]),
 `cpu_baseline`.
+
+--dump-outputs DIR writes what the last timed step returned (the .bz2 stream, sampled) as .npy files under DIR, so
+that the streams of two builds can be compared; see dump_outputs().
 """
 import argparse
 import ctypes as C
@@ -27,6 +30,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark writes nothing into the tree it runs from, which may be read-only
 
 import numpy as np  # noqa: E402
 
@@ -34,6 +38,7 @@ SEED = 20260923
 LEVEL = 9
 METRIC = "bzip2_-9_encode_MBps"
 BS9 = LEVEL * 100000 - 19
+DUMP_HEAD, DUMP_TAIL, DUMP_SAMPLE = 1 << 20, 1 << 16, 4 << 20   # stream bytes --dump-outputs keeps
 
 
 def gen_ascii(nbytes, seed):
@@ -328,6 +333,30 @@ def bwtc_leg(L, _native, torch, host, mb, check_blocks):
     return res
 
 
+def dump_outputs(path, d_stream, n):
+    """The .bz2 stream of the last timed step (first n bytes of the CUDA tensor d_stream) as .npy files under `path`:
+    its length, its first MiB and last 64 KiB (header, first blocks, last block, stream CRC) and its bytes at up to
+    4 Mi positions drawn with PCG64(SEED) (every position of a shorter stream), with those positions.  Byte values are
+    float32, the length and positions float64 (exact below 2**53): about 52 MB in all.  The same arguments give the
+    same input, so two builds are compared file by file."""
+    import torch
+    os.makedirs(path, exist_ok=True)
+    s = d_stream[:n]
+    if n <= DUMP_SAMPLE:
+        idx = np.arange(n)
+    else:
+        idx = np.unique(np.random.Generator(np.random.PCG64(SEED)).integers(0, n, size=DUMP_SAMPLE))
+    arrays = {
+        "stream_length": np.array([n], dtype=np.float64),
+        "stream_head": s[:DUMP_HEAD].cpu().numpy().astype(np.float32),
+        "stream_tail": s[max(0, n - DUMP_TAIL):].cpu().numpy().astype(np.float32),
+        "stream_sample_index": idx.astype(np.float64),
+        "stream_sample": s[torch.from_numpy(idx).to(s.device)].cpu().numpy().astype(np.float32),
+    }
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -338,6 +367,7 @@ def main():
     ap.add_argument("--no-cpu", action="store_true", help="skip every leg that runs the CPU oracle (cpu_baseline, parity)")
     ap.add_argument("--no-extra", action="store_true", help="skip the config3 and bwtc legs")
     ap.add_argument("--bwtc-mb", type=int, default=int(os.environ.get("B2_BENCH_BWTC_MB", "64")), help="MiB of the config-2 buffer for the BWTC leg (config 4 = 1024)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the stream of the last timed step (sampled) to DIR/*.npy")
     args = ap.parse_args()
     if args.impl == "reference":
         return run_reference(args)
@@ -454,6 +484,14 @@ def main():
     clocks = sampler.stop(t0, t0 + wall) if rank == 0 else None
     comp_bytes = state["comp"]
     trace = _native.last_trace() if world == 1 else []
+    if args.dump_outputs:
+        if world == 1:
+            dump_outputs(args.dump_outputs, d_out, comp_bytes)
+        else:
+            full = state["ss"].gather()   # collective: the last timed step's stream, assembled on rank 0
+            if rank == 0:
+                dump_outputs(args.dump_outputs, full, full.numel())
+            del full
 
     # device time: max over ranks (events on the library's launching stream)
     t = torch.tensor([dev_ms, wall * 1e3], dtype=torch.float64, device="cuda")

@@ -1,6 +1,6 @@
 """Generates tests/golden/golden.json: outputs of the CPU oracle (oracle/bz2_oracle.c) on the
-reference's own test inputs (/root/reference/test/sample*.ref).  The reference is JavaScript and
-cannot run in this image, so these are the pinned outputs of its restatement; sizes in legacy-sort
+reference's own test inputs (its test/sample*.ref, stored under tests/golden/fixtures).  These are the
+pinned outputs of the oracle, the C restatement of the reference's JavaScript; sizes in legacy-sort
 mode equal README.md:42,45 of the reference.  Run:  python tests/golden/make_golden.py
 """
 import hashlib
@@ -11,12 +11,12 @@ import sys
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 sys.path.insert(0, ROOT)
 from oracle import oracle as O  # noqa: E402
+from tests.util import fixture  # noqa: E402
 
-REF = "/root/reference/test"
 out = {}
 for k in range(6):
     name = "sample%d" % k
-    data = open(os.path.join(REF, name + ".ref"), "rb").read()
+    data = fixture(name + ".ref")
     out["ref_%s" % name] = {"size": len(data), "sha256": hashlib.sha256(data).hexdigest()}
     for lv in (1, 9):
         z, tr = O.bzip2_compress(data, lv, trace=True)
@@ -28,7 +28,7 @@ for k in range(6):
         z = O.bwtc_compress(data, lv)
         out["bwtc_%s_-%d" % (name, lv)] = {"size": len(z), "sha256": hashlib.sha256(z).hexdigest()}
 for lv in (1, 9):
-    z = O.bzip2_compress(open(os.path.join(REF, "sample5.ref"), "rb").read(), lv, legacy_sort=True)
+    z = O.bzip2_compress(fixture("sample5.ref"), lv, legacy_sort=True)
     out["bzip2_sample5_-%d_legacy_v8_sort" % lv] = {"size": len(z), "sha256": hashlib.sha256(z).hexdigest()}
 json.dump(out, open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden.json"), "w"), indent=1, sort_keys=True)
 print("wrote", len(out), "entries")

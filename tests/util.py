@@ -1,23 +1,40 @@
 """Shared helpers for the test-suite: fixtures, synthetic inputs, native bindings."""
+import bz2
 import ctypes as C
+import functools
+import hashlib
+import json
+import lzma
 import os
 
 import numpy as np
-import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-_FIX_DIRS = [os.path.join(ROOT, "oracle", "_ref", "fixtures"), "/root/reference/test"]
+GOLDEN = os.path.join(ROOT, "tests", "golden")
 
 
+@functools.lru_cache(maxsize=None)
 def fixture(name):
-    """Reference test fixture (test/sample*.ref, *.bz2, *.bzt ...).  They are not copied into git:
-    __graft_entry__.build() mirrors them into oracle/_ref/fixtures (git-ignored, travels to the GPU box)."""
-    for d in _FIX_DIRS:
-        p = os.path.join(d, name)
-        if os.path.exists(p):
-            with open(p, "rb") as f:
-                return f.read()
-    pytest.skip("reference fixture %s not available" % name)
+    """The reference's test fixture `name` (its test/sample*.ref, *.bz2, *.bzt and block files), rebuilt from
+    tests/golden/fixtures as tests/golden/fixtures.json describes: the .ref texts are stored xz-compressed and the
+    .bzt tables as they are; every .bz2 of the reference is libbz2's stream of its .ref at the level in its header, and
+    a block file is a slice of its .ref.  The result must have the size and SHA-256 of the reference's file."""
+    with open(os.path.join(GOLDEN, "fixtures.json")) as f:
+        spec = json.load(f)[name]
+    path = os.path.join(GOLDEN, "fixtures", name)
+    if "bzip2_level" in spec:
+        data = bz2.compress(fixture(spec["from"]), spec["bzip2_level"])
+    elif "offset" in spec:
+        data = fixture(spec["from"])[spec["offset"]:spec["offset"] + spec["size"]]
+    elif os.path.exists(path + ".xz"):
+        with open(path + ".xz", "rb") as f:
+            data = lzma.decompress(f.read())
+    else:
+        with open(path, "rb") as f:
+            data = f.read()
+    got = (len(data), hashlib.sha256(data).hexdigest())
+    assert got == (spec["size"], spec["sha256"]), "fixture %s rebuilt as %r, not the reference's file" % (name, got)
+    return data
 
 
 def rng(seed):

@@ -6,6 +6,7 @@ config 3: "enwik8-shaped" text: order-3 byte Markov chain trained on the referen
           (copy 200-5000 bytes from >= 64 KiB back).  Vectorised: many independent chains are advanced in
           lock-step and concatenated, which keeps the order-3 statistics and is fast enough for 100 MB.
 """
+import lzma
 import os
 import numpy as np
 
@@ -13,10 +14,9 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 def _train_bytes():
-    for p in (os.path.join(ROOT, "oracle", "_ref", "fixtures", "sample5.ref"), "/root/reference/test/sample5.ref"):
-        if os.path.exists(p):
-            return np.frombuffer(open(p, "rb").read(), dtype=np.uint8)
-    raise FileNotFoundError("sample5.ref (reference fixture) not found: run __graft_entry__.build() where /root/reference exists")
+    # the reference's test/sample5.ref, kept xz-compressed with the test fixtures
+    with open(os.path.join(ROOT, "tests", "golden", "fixtures", "sample5.ref.xz"), "rb") as f:
+        return np.frombuffer(lzma.decompress(f.read()), dtype=np.uint8)
 
 
 def enwik_like(nbytes, seed=20260923, chains=4096):
